@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Jacobi pressure-solve throughput (BASELINE.json metric) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the metric's hot path over one batch of synthetic input: the pressure
 solve of step() — clear (p <- PRESSURE*p, S:1253-1257) + PRESSURE_ITERATIONS Jacobi sweeps
@@ -22,6 +22,11 @@ per-pass figures of a whole step().
 `--impl reference`: the reference cannot run here (browser + WebGL, SURVEY §0.4), so the reference
 arm is the CPU restatement of script.js (oracle/, kind "port") on the host cores this process may
 use (affinity mask capped by the cgroup quota), buffers first-touched by the threads that sweep them.
+`--dump-outputs DIR`: after the timed steps, the pressure field the last timed step left is written to
+DIR/pressure.npy (float32; at N>1 DIR/pressure_rank<r>.npy, each rank its own rows), so that two builds
+can be compared output for output on the same seeded inputs.  A field larger than the 32 MiB budget
+(shared by the ranks) is cut to a fixed, seeded sample of its rows, whose indices go to
+DIR/<name>_rows.npy (float64).
 """
 from __future__ import annotations
 
@@ -169,6 +174,21 @@ def crc(a: np.ndarray) -> int:
     return zlib.crc32(np.ascontiguousarray(a).view(np.uint8).reshape(-1).data)
 
 
+DUMP_BYTES = 32 << 20     # --dump-outputs budget over all ranks
+
+
+def dump_field(out_dir, name, a, budget):
+    """a -> out_dir/name.npy as float32; above `budget` bytes only a fixed, seeded sample of its rows
+    (sorted), with their indices in out_dir/name_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    if a.nbytes > budget:
+        k = max(1, budget // a[0].nbytes)
+        rows = np.sort(np.random.default_rng(0).choice(a.shape[0], k, replace=False))
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        a = a[rows]
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 # ---- CPU legs -------------------------------------------------------------------------------------
 
 class CpuSolve:
@@ -224,6 +244,8 @@ def run_reference(args, rank, world):
     for _ in range(args.steps):
         t0 = time.perf_counter(); c.sweeps(sweeps); per.append(time.perf_counter() - t0)
     dt = time.perf_counter() - t_all
+    if args.dump_outputs:
+        dump_field(args.dump_outputs, "pressure", c.p, DUMP_BYTES)
     val = W * H * sweeps * args.steps / dt
     rates = [W * H * sweeps / t for t in per]
     sample = f"each step = {sweeps} Jacobi sweeps of {W}x{H} fp32 out of the {ITERS}-sweep solve"
@@ -285,7 +307,10 @@ def main():
     ap.add_argument("--grid", type=int, default=4096, help="square grid size of the workload (BASELINE configs: 4096 / 8192 / 16384)")
     ap.add_argument("--iters", type=int, default=50, help="Jacobi iterations per solve (BASELINE configs: 50 / 40 / 80)")
     ap.add_argument("--strong", action="store_true", help="N>1: the headline `value` is measured on ONE grid x grid domain split into N row slabs (default: weak, one grid x grid slab per GPU, plus a `strong` block)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the pressure field of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     global W, H, ITERS
     W = H = args.grid
@@ -387,6 +412,8 @@ def main():
         clk.reset()                       # keep only the samples taken during the timed region
         ms = time_steps(sim, solve, args.steps, tag="solve", align=world > 1)
         sim.sync()
+        # read before the extra solves below overwrite it; written once the clock sampler has stopped
+        dumped = sim.readField("pressure") if args.dump_outputs else None
         # keep the device loaded until NVML has a few samples even if the timed region is short
         # (single GPU only: on slabs every solve is a collective, so all ranks must issue the
         # same number of them; there a fixed number of extra solves keeps the sampler fed)
@@ -398,6 +425,9 @@ def main():
             for _ in range(20):
                 solve()
             sim.sync()
+    if dumped is not None:
+        dump_field(args.dump_outputs, "pressure" if world == 1 else f"pressure_rank{rank}", dumped, DUMP_BYTES // world)
+        del dumped
     barrier()
     # exact launch counts of the timed region: kernels per solve x steps, Jacobi kernels separately
     l1, j1, h1 = sim.launch_count(), sim.stat("jacobi_launches"), sim.stat("halo_launches")

@@ -2,6 +2,7 @@
 
 Run in the build container only (needs /root/reference/script.js):
     python tests/golden/make_golden.py
+    python tests/golden/make_golden.py citations    # script_js_citations.json only
 The .npz files are committed; the tests never read /root/reference.
 Inputs are seeded; every file stores inputs and the reference-shader outputs, fp32 storage,
 `!supportLinearFiltering` path (MANUAL_FILTERING + NEAREST samplers: arithmetic fully defined by the
@@ -143,7 +144,24 @@ def resample(name, Ws, Hs, Wd, Hd, ch, seed):
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **o)
 
 
+def citations():
+    """script_js_citations.json for tests/test_citations_and_plan.py: the line count of script.js and
+    the 1-based lines on which each of that test's spot-check needles occurs (no script.js text)."""
+    import json
+    sys.path.insert(0, os.path.dirname(OUT))
+    from test_citations_and_plan import SPOT_CHECKS
+    js = open(G.REFERENCE_JS).read().splitlines()
+    needles = sorted({needle for _, _, needle in SPOT_CHECKS})
+    ref = {"lines": len(js), "needle_lines": {s: [k + 1 for k, l in enumerate(js) if s in l] for s in needles}}
+    with open(os.path.join(OUT, "script_js_citations.json"), "w") as f:
+        json.dump(ref, f, indent=1)
+        f.write("\n")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "citations":
+        citations()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "r02":     # the vectors added in round 2 only
         resample("resample_v_32_to_48", 32, 32, 48, 48, 2, 31)           # up-sample, ragged ratio
         resample("resample_dye_64_to_32", 64, 64, 32, 32, 4, 32)         # down-sample by 2 (power of two)

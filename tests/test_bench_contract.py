@@ -5,7 +5,24 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
+from conftest import bits_equal
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def bench(*args):
+    return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                          timeout=600, cwd=ROOT)
+
+
+def synth_inputs(grid):
+    """bench.synth_inputs() at grid x grid: pressure and divergence from seed 42."""
+    rng = np.random.default_rng(42)
+    d = rng.uniform(-1, 1, (grid, grid)).astype(np.float32)
+    return rng.standard_normal((grid, grid)).astype(np.float32), d
 
 
 def test_reference_arm_prints_the_contract_line():
@@ -33,3 +50,42 @@ def test_gpu_arm_refuses_to_run_without_a_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"],
                          capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert out.returncode != 0 and "no CPU path" in (out.stderr + out.stdout)
+
+
+@pytest.mark.parametrize("grid,sampled", [(512, False), (4096, True)])
+def test_reference_arm_dumps_its_last_timed_step(oracle, tmp_path, grid, sampled):
+    """--dump-outputs on the CPU arm: 3 warm-up steps of 2 sweeps and 2 timed steps of 10 sweeps leave the
+    oracle's 26 sweeps of the seeded inputs; a 4096^2 field is over the budget and cut to seeded rows."""
+    out = bench("--impl", "reference", "--steps", "2", "--warmup", "1", "--grid", str(grid),
+                "--dump-outputs", str(tmp_path))
+    assert out.returncode == 0, out.stderr[-2000:]
+    p, d = synth_inputs(grid)
+    want = oracle.jacobi(p, d, 2 * 3 + 10 * 2)
+    got = np.load(tmp_path / "pressure.npy")
+    assert got.dtype == np.float32
+    if sampled:
+        rows = np.load(tmp_path / "pressure_rows.npy")
+        assert rows.dtype == np.float64 and np.all(np.diff(rows) > 0) and got.nbytes <= 32 << 20
+        want = want[rows.astype(np.int64)]
+    else:
+        assert not (tmp_path / "pressure_rows.npy").exists()
+    assert bits_equal(got, want)
+
+
+def test_steps_below_one_are_refused():
+    out = bench("--impl", "reference", "--steps", "0", "--grid", "512")
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_its_last_timed_step(oracle, tmp_path):
+    """--dump-outputs on the timed path: 3 warm-up and 4 timed solves (each clear + 50 Jacobi sweeps), so the
+    dump is the oracle's 7th solve of the seeded inputs, bit for bit."""
+    out = bench("--steps", "4", "--warmup", "3", "--grid", "512", "--iters", "50", "--quick",
+                "--dump-outputs", str(tmp_path))
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])["steps"] == 4
+    p, d = synth_inputs(512)
+    for _ in range(3 + 4):
+        p = oracle.jacobi(oracle.clear(p, 0.8), d, 50)
+    assert bits_equal(np.load(tmp_path / "pressure.npy"), p)

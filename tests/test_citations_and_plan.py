@@ -1,15 +1,25 @@
 """Housekeeping that needs no GPU: (1) every `S:n[-m]` citation in the product, oracle and docs points
-inside /root/reference/script.js and, for the shader / function cites in include/fluid.h, at the
-construct it names (skipped where the reference is not mounted, e.g. on the GPU box);
+inside the reference's script.js and, for the shader / function cites in include/fluid.h, at the
+construct it names (against tests/golden/script_js_citations.json: the line count of script.js and
+the lines on which each spot-check needle occurs, cut by tests/golden/make_golden.py citations);
 (2) randomised invariants of the slab plan."""
+import json
 import os
 import re
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/script.js"
+REF_LINES = os.path.join(ROOT, "tests", "golden", "script_js_citations.json")
+# (first line, last line, text that must occur on one of them) in script.js
+SPOT_CHECKS = [
+    (1231, 1294, "function step (dt)"), (1441, 1455, "function splat (x, y, dx, dy, color)"),
+    (868, 890, "pressureShader"), (1259, 1266, "PRESSURE_ITERATIONS"),
+    (746, 784, "advectionShader"), (786, 812, "divergenceShader"), (814, 833, "curlShader"),
+    (835, 866, "vorticityShader"), (892, 913, "gradientSubtractShader"), (726, 744, "splatShader"),
+    (508, 519, "clearShader"), (982, 1010, "function initFramebuffers"), (1612, 1624, "function getResolution"),
+    (549, 612, "displayShaderSource"), (1296, 1317, "function render (target)"),
+]
 FILES = ["include/fluid.h", "DESIGN.md", "INTEGRATION.md", "oracle/fluid_oracle.c", "oracle/fluid_oracle.h",
          "oracle/glsl_exec.py", "webgl_fluid_simulation_b200/sim.py", "webgl_fluid_simulation_b200/js/fluid-sim.js",
          "webgl_fluid_simulation_b200/csrc/jacobi.cuh", "webgl_fluid_simulation_b200/csrc/passes.cuh",
@@ -18,23 +28,16 @@ FILES = ["include/fluid.h", "DESIGN.md", "INTEGRATION.md", "oracle/fluid_oracle.
          "webgl_fluid_simulation_b200/napi/fluid_napi.c", "README.md"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference not mounted")
 def test_script_js_citations_are_in_range_and_on_target():
-    js = open(REF).read().splitlines()
-    n = len(js)
+    ref = json.load(open(REF_LINES))
+    n = ref["lines"]
     for f in FILES:
         for m in re.finditer(r"\bS:(\d+)(?:-(\d+))?", open(os.path.join(ROOT, f)).read()):
             a = int(m.group(1)); b = int(m.group(2) or a)
             assert 1 <= a <= b <= n, (f, m.group(0))
     # spot-check that the headline cites land on what they claim
-    def has(lo, hi, needle):
-        return any(needle in l for l in js[lo - 1:hi])
-    assert has(1231, 1294, "function step (dt)") and has(1441, 1455, "function splat (x, y, dx, dy, color)")
-    assert has(868, 890, "pressureShader") and has(1259, 1266, "PRESSURE_ITERATIONS")
-    assert has(746, 784, "advectionShader") and has(786, 812, "divergenceShader") and has(814, 833, "curlShader")
-    assert has(835, 866, "vorticityShader") and has(892, 913, "gradientSubtractShader") and has(726, 744, "splatShader")
-    assert has(508, 519, "clearShader") and has(982, 1010, "function initFramebuffers") and has(1612, 1624, "function getResolution")
-    assert has(549, 612, "displayShaderSource") and has(1296, 1317, "function render (target)")
+    for lo, hi, needle in SPOT_CHECKS:
+        assert any(lo <= k <= hi for k in ref["needle_lines"][needle]), (lo, hi, needle)
 
 
 def test_slab_plan_invariants_randomised():
