@@ -80,7 +80,8 @@ typedef enum fluid_param {
 #define FLUID_FLAG_HALF_STORAGE 0x10u /* store every field as fp16 like the reference's textures (S:138-147,
                                          S:986-1006): fp32 arithmetic, round-to-nearest-even on every pass
                                          write, one launch per reference blit; single GPU; the ABI still
-                                         speaks fp32 (fluid_read widens, fluid_write narrows)              */
+                                         speaks fp32 (fluid_read widens, fluid_write narrows).
+                                         fluid_render_postfx then uses fp16 post-FX FBOs as well     */
 #define FLUID_FLAG_TILED_PASSES 0x8u /* generation-1 kernels (one thread per fragment / smem tile) for
                                         curl-vorticity-divergence and gradientSubtract instead of the
                                         row-streaming ones (comparison + fallback path)              */
@@ -223,7 +224,11 @@ int fluid_render_band(fluid_t* h, int height, int* y0, int* y1);
  * keywords.  fx = the BLOOM_* / SUNRAYS_* keys of `config`; dither_rgb = the dw x dh RGB dithering
  * texture (LDR_LLL1_0.png / 255, first image row first, S:1128-1158).  host_bloom (bloom FBO,
  * getResolution(BLOOM_RESOLUTION) x RGBA) and host_sunrays (getResolution(SUNRAYS_RESOLUTION) x R)
- * may be NULL. */
+ * may be NULL.  The sunrays mask is drawn into dye.write, like the reference (S:1300); dye.read is
+ * untouched.  On a FLUID_FLAG_HALF_STORAGE handle the bloom FBO, the bloom pyramid, both sunrays
+ * FBOs and the mask are fp16, as the reference creates them (S:1012-1043): every blit rounds its
+ * output to fp16 (RN-even), and host_bloom / host_sunrays come back widened to fp32 (exactly).  The
+ * dithering texture and host_rgba are fp32 in both modes.  Not available on slab handles. */
 typedef struct fluid_postfx {
     int32_t bloom_iterations;    /* S:77 default 8    */
     int32_t bloom_resolution;    /* S:78 default 256  */

@@ -15,6 +15,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "jacobi.cuh"
@@ -779,6 +780,103 @@ int create_common(const fluid_config* cfg, int rank, int world, const void* uid,
     int rc = body();
     if (rc != FLUID_OK) { g_create_error = h->err; fluid_destroy(h); return rc; }
     *out = h;
+    return FLUID_OK;
+}
+
+// createFBO's clear to (0,0,0,1) (S:1059) of the bloom FBO, for either storage
+inline void clear_fbo(float4* p, size_t n, cudaStream_t s) { fill_alpha_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(p, n); }
+inline void clear_fbo(hs::h4* p, size_t n, cudaStream_t s) { hs::fill_alpha_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(p, n); }
+
+// The post-FX chain of fluid_render_postfx on T4 / T1 textures: float4 / float for fp32 storage,
+// hs::h4 / hs::h1 for FLUID_FLAG_HALF_STORAGE, where (as in the reference, S:1012-1043 and S:1300)
+// the bloom FBO, the pyramid, both sunrays FBOs and the mask in dye.write are fp16.  `tmp` collects
+// the per-call device allocations; the caller frees them.
+template <typename T4, typename T1>
+int render_postfx_chain(fluid_t* h, int width, int height, const fluid_postfx* fx, const float* dither_rgb, int dw, int dh,
+                        float back_r, float back_g, float back_b, float* host_rgba, float* host_bloom, float* host_sunrays,
+                        int bw, int bh, int sw, int sh, std::vector<void*>& tmp) {
+    constexpr bool half = !std::is_same<T4, float4>::value;
+    auto dalloc = [&](size_t bytes) -> void* { void* p = nullptr; if (cudaMalloc(&p, bytes) != cudaSuccess) return nullptr; tmp.push_back(p); return p; };
+    const size_t cells = (size_t)width * height;
+    if (cells > h->frame_cells) {
+        CU(cudaStreamSynchronize(h->stream));
+        cudaFree(h->frame); h->frame = nullptr; h->frame_cells = 0;
+        CU(cudaMalloc((void**)&h->frame, cells * sizeof(float4)));
+        h->frame_cells = cells;
+    }
+    const int Wd = h->cfg.dye_w, Hd = h->cfg.dye_h;
+    const T4* dye = (const T4*)h->dye.read;
+    dim3 b(32, 8);
+    T4* bloom = (T4*)dalloc((size_t)bw * bh * sizeof(T4));
+    T1* sun = (T1*)dalloc((size_t)sw * sh * sizeof(T1));
+    T1* sun2 = (T1*)dalloc((size_t)sw * sh * sizeof(T1));
+    float* dith = (float*)dalloc((size_t)dw * dh * 3 * sizeof(float));
+    if (!bloom || !sun || !sun2 || !dith) return fail(h, FLUID_ERR_NOMEM, "out of device memory for the post-FX targets");
+    // fp16 storage: host_bloom / host_sunrays are the fp16 textures widened (exactly) on the device
+    float* wide_bloom = nullptr; float* wide_sun = nullptr;
+    if (half && host_bloom && !(wide_bloom = (float*)dalloc((size_t)bw * bh * 4 * sizeof(float))))
+        return fail(h, FLUID_ERR_NOMEM, "out of device memory for the bloom read-back");
+    if (half && host_sunrays && !(wide_sun = (float*)dalloc((size_t)sw * sh * sizeof(float))))
+        return fail(h, FLUID_ERR_NOMEM, "out of device memory for the sunrays read-back");
+    CU(cudaMemcpyAsync(dith, dither_rgb, (size_t)dw * dh * 3 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    clear_fbo(bloom, (size_t)bw * bh, h->stream);
+    // ---- applyBloom(dye.read, bloom) ----------------------------------------------------------
+    struct Lv { T4* p; int w, h; };
+    std::vector<Lv> pyr;
+    for (int i = 0; i < fx->bloom_iterations; ++i) {
+        const int pw = bw >> (i + 1), ph = bh >> (i + 1);
+        if (pw < 2 || ph < 2) break;
+        T4* p = (T4*)dalloc((size_t)pw * ph * sizeof(T4));
+        if (!p) return fail(h, FLUID_ERR_NOMEM, "out of device memory for the bloom pyramid");
+        pyr.push_back({p, pw, ph});
+    }
+    int nk = 1;
+    if (pyr.size() >= 2) {
+        const double knee = fx->bloom_threshold * fx->bloom_soft_knee + 0.0001;
+        bloom_prefilter_kernel<<<grid2d(bw, bh, b), b, 0, h->stream>>>(
+            dye, Wd, Hd, bloom, bw, bh, (float)(fx->bloom_threshold - knee),
+            (float)(knee * 2), (float)(0.25 / knee), (float)fx->bloom_threshold);
+        ++nk;
+        Lv last{bloom, bw, bh};
+        for (auto& d : pyr) {
+            box4_kernel<<<grid2d(d.w, d.h, b), b, 0, h->stream>>>(last.p, last.w, last.h, d.p, d.w, d.h, 1.0f, 0);
+            last = d; ++nk;
+        }
+        for (int i = (int)pyr.size() - 2; i >= 0; --i) {
+            box4_kernel<<<grid2d(pyr[i].w, pyr[i].h, b), b, 0, h->stream>>>(last.p, last.w, last.h, pyr[i].p, pyr[i].w, pyr[i].h, 1.0f, 1);
+            last = pyr[i]; ++nk;
+        }
+        box4_kernel<<<grid2d(bw, bh, b), b, 0, h->stream>>>(last.p, last.w, last.h, bloom, bw, bh, (float)fx->bloom_intensity, 0);
+        ++nk;
+    }
+    // ---- applySunrays(dye.read, dye.write, sunrays); blur(sunrays, sunraysTemp, 1) ---------------
+    sunrays_mask_kernel<<<grid2d(Wd, Hd, b), b, 0, h->stream>>>(dye, (T4*)h->dye.write, Wd, Hd);
+    sunrays_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>((const T4*)h->dye.write, Wd, Hd, sun, sw, sh, (float)fx->sunrays_weight);
+    blur3_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>(sun, sun2, sw, sh, (float)(1.0 / (double)sw), 0.0f);
+    blur3_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>(sun2, sun, sw, sh, 0.0f, (float)(1.0 / (double)sh));
+    // ---- drawColor + drawDisplay ---------------------------------------------------------------------
+    display_full_kernel<<<grid2d(width, height, b), b, 0, h->stream>>>(
+        dye, Wd, Hd, bloom, bw, bh, sun, sw, sh, dith, dw, dh, h->frame, width, height,
+        back_r, back_g, back_b, h->background, h->cfg.aspect,
+        make_float4((float)(1.0 / (double)width), (float)(1.0 / (double)height), (float)((double)width / (double)dw), (float)((double)height / (double)dh)));
+    nk += 5;
+    const float* out_bloom = (const float*)bloom;
+    const float* out_sun = (const float*)sun;
+    if (wide_bloom) {
+        const size_t n = (size_t)bw * bh * 4;
+        hs::widen_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((const hs::h1*)bloom, wide_bloom, n);
+        out_bloom = wide_bloom; ++nk;
+    }
+    if (wide_sun) {
+        const size_t n = (size_t)sw * sh;
+        hs::widen_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((const hs::h1*)sun, wide_sun, n);
+        out_sun = wide_sun; ++nk;
+    }
+    int r = check_launch(h, "post-FX kernels", nk); if (r) return r;
+    CU(cudaMemcpyAsync(host_rgba, h->frame, cells * sizeof(float4), cudaMemcpyDeviceToHost, h->stream));
+    if (host_bloom) CU(cudaMemcpyAsync(host_bloom, out_bloom, (size_t)bw * bh * 4 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    if (host_sunrays) CU(cudaMemcpyAsync(host_sunrays, out_sun, (size_t)sw * sh * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
     return FLUID_OK;
 }
 
@@ -1719,7 +1817,6 @@ int fluid_render_postfx(fluid_t* h, int width, int height, const fluid_postfx* f
     if (!h || !fx || !dither_rgb || !host_rgba || width < 1 || height < 1 || dw < 1 || dh < 1)
         return fail(h, FLUID_ERR_INVALID, "bad argument");
     if (h->slab()) return not_on_slab(h, "fluid_render_postfx");
-    if (h->half) return fail(h, FLUID_ERR_INVALID, "fluid_render_postfx is not built for FLUID_FLAG_HALF_STORAGE (the reference's bloom / sunrays FBOs are fp16 too)");
     const size_t cells = (size_t)width * height;
     if (n_floats != 4 * cells) return fail(h, FLUID_ERR_INVALID, "render target has %zu floats, caller passed %zu", 4 * cells, n_floats);
     int bw, bh, sw, sh;
@@ -1727,73 +1824,13 @@ int fluid_render_postfx(fluid_t* h, int width, int height, const fluid_postfx* f
     fluid_get_resolution(fx->sunrays_resolution, width, height, &sw, &sh);
     if (bw < 1 || bh < 1 || sw < 1 || sh < 1) return fail(h, FLUID_ERR_INVALID, "bad post-FX resolution");
     std::vector<void*> tmp;
-    auto dalloc = [&](size_t bytes) -> void* { void* p = nullptr; if (cudaMalloc(&p, bytes) != cudaSuccess) return nullptr; tmp.push_back(p); return p; };
-    auto cleanup = [&]() { cudaStreamSynchronize(h->stream); for (void* p : tmp) cudaFree(p); };
-    int rc = FLUID_OK;
-    auto body = [&]() -> int {
-        if (cells > h->frame_cells) {
-            CU(cudaStreamSynchronize(h->stream));
-            cudaFree(h->frame); h->frame = nullptr; h->frame_cells = 0;
-            CU(cudaMalloc((void**)&h->frame, cells * sizeof(float4)));
-            h->frame_cells = cells;
-        }
-        const int Wd = h->cfg.dye_w, Hd = h->cfg.dye_h;
-        dim3 b(32, 8);
-        float4* bloom = (float4*)dalloc((size_t)bw * bh * sizeof(float4));
-        float* sun = (float*)dalloc((size_t)sw * sh * sizeof(float));
-        float* sun2 = (float*)dalloc((size_t)sw * sh * sizeof(float));
-        float* dith = (float*)dalloc((size_t)dw * dh * 3 * sizeof(float));
-        if (!bloom || !sun || !sun2 || !dith) return fail(h, FLUID_ERR_NOMEM, "out of device memory for the post-FX targets");
-        CU(cudaMemcpyAsync(dith, dither_rgb, (size_t)dw * dh * 3 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-        fill_alpha_kernel<<<(unsigned)(((size_t)bw * bh + 255) / 256), 256, 0, h->stream>>>(bloom, (size_t)bw * bh);   // createFBO clear
-        // ---- applyBloom(dye.read, bloom) ----------------------------------------------------------
-        struct Lv { float4* p; int w, h; };
-        std::vector<Lv> pyr;
-        for (int i = 0; i < fx->bloom_iterations; ++i) {
-            const int pw = bw >> (i + 1), ph = bh >> (i + 1);
-            if (pw < 2 || ph < 2) break;
-            float4* p = (float4*)dalloc((size_t)pw * ph * sizeof(float4));
-            if (!p) return fail(h, FLUID_ERR_NOMEM, "out of device memory for the bloom pyramid");
-            pyr.push_back({p, pw, ph});
-        }
-        int nk = 1;
-        if (pyr.size() >= 2) {
-            const double knee = fx->bloom_threshold * fx->bloom_soft_knee + 0.0001;
-            bloom_prefilter_kernel<<<grid2d(bw, bh, b), b, 0, h->stream>>>(
-                (const float4*)h->dye.read, Wd, Hd, bloom, bw, bh, (float)(fx->bloom_threshold - knee),
-                (float)(knee * 2), (float)(0.25 / knee), (float)fx->bloom_threshold);
-            ++nk;
-            Lv last{bloom, bw, bh};
-            for (auto& d : pyr) {
-                box4_kernel<<<grid2d(d.w, d.h, b), b, 0, h->stream>>>(last.p, last.w, last.h, d.p, d.w, d.h, 1.0f, 0);
-                last = d; ++nk;
-            }
-            for (int i = (int)pyr.size() - 2; i >= 0; --i) {
-                box4_kernel<<<grid2d(pyr[i].w, pyr[i].h, b), b, 0, h->stream>>>(last.p, last.w, last.h, pyr[i].p, pyr[i].w, pyr[i].h, 1.0f, 1);
-                last = pyr[i]; ++nk;
-            }
-            box4_kernel<<<grid2d(bw, bh, b), b, 0, h->stream>>>(last.p, last.w, last.h, bloom, bw, bh, (float)fx->bloom_intensity, 0);
-            ++nk;
-        }
-        // ---- applySunrays(dye.read, dye.write, sunrays); blur(sunrays, sunraysTemp, 1) ---------------
-        sunrays_mask_kernel<<<grid2d(Wd, Hd, b), b, 0, h->stream>>>((const float4*)h->dye.read, (float4*)h->dye.write, Wd, Hd);
-        sunrays_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>((const float4*)h->dye.write, Wd, Hd, sun, sw, sh, (float)fx->sunrays_weight);
-        blur3_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>(sun, sun2, sw, sh, (float)(1.0 / (double)sw), 0.0f);
-        blur3_kernel<<<grid2d(sw, sh, b), b, 0, h->stream>>>(sun2, sun, sw, sh, 0.0f, (float)(1.0 / (double)sh));
-        // ---- drawColor + drawDisplay ---------------------------------------------------------------------
-        display_full_kernel<<<grid2d(width, height, b), b, 0, h->stream>>>(
-            (const float4*)h->dye.read, Wd, Hd, bloom, bw, bh, sun, sw, sh, dith, dw, dh, h->frame, width, height,
-            back_r, back_g, back_b, h->background, h->cfg.aspect,
-            make_float4((float)(1.0 / (double)width), (float)(1.0 / (double)height), (float)((double)width / (double)dw), (float)((double)height / (double)dh)));
-        int r = check_launch(h, "post-FX kernels", nk + 5); if (r) return r;
-        CU(cudaMemcpyAsync(host_rgba, h->frame, cells * sizeof(float4), cudaMemcpyDeviceToHost, h->stream));
-        if (host_bloom) CU(cudaMemcpyAsync(host_bloom, bloom, (size_t)bw * bh * sizeof(float4), cudaMemcpyDeviceToHost, h->stream));
-        if (host_sunrays) CU(cudaMemcpyAsync(host_sunrays, sun, (size_t)sw * sh * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-        CU(cudaStreamSynchronize(h->stream));
-        return FLUID_OK;
-    };
-    rc = body();
-    cleanup();
+    const int rc = h->half
+        ? render_postfx_chain<hs::h4, hs::h1>(h, width, height, fx, dither_rgb, dw, dh, back_r, back_g, back_b, host_rgba,
+                                              host_bloom, host_sunrays, bw, bh, sw, sh, tmp)
+        : render_postfx_chain<float4, float>(h, width, height, fx, dither_rgb, dw, dh, back_r, back_g, back_b, host_rgba,
+                                             host_bloom, host_sunrays, bw, bh, sw, sh, tmp);
+    cudaStreamSynchronize(h->stream);
+    for (void* p : tmp) cudaFree(p);
     return rc;
 }
 

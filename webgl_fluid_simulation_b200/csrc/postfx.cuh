@@ -6,22 +6,65 @@
 // GL_LINEAR formula of passes.cuh (linear_fetch4).  Arithmetic order follows the GLSL; with the
 // library's --fmad=false / IEEE div+sqrt build everything is bit-identical to the CPU oracle except
 // the display's pow() (linearToGamma), which is tolerance-checked like splat's exp().
+//
+// The kernels are templated over the texture storage: float4 / float (fp32 storage) or hs::h4 /
+// hs::h1 (FLUID_FLAG_HALF_STORAGE).  The reference creates the bloom FBO, the bloom pyramid and both
+// sunrays FBOs with ext.halfFloatTexType (S:1012-1043) and draws the mask into the RGBA16F dye.write
+// (S:1300), so in that mode every texel is widened exactly when fetched and every blit's output is
+// rounded to fp16 (RN-even, hs::st) when stored; the arithmetic in between is the same fp32 code.
+// The dithering texture and the final target are fp32 in both modes.
 #pragma once
 #include <cuda_runtime.h>
 
+#include "half_passes.cuh"
 #include "passes.cuh"
 
 namespace fk {
 
-__device__ __forceinline__ float linear_fetch1(const float* __restrict__ tex, int W, int H, float uvx, float uvy) {
+// texel access by storage type: fp32 as stored; fp16 widened exactly / rounded to nearest even
+__device__ __forceinline__ float tex_ld(const float* __restrict__ t, size_t k) { return __ldg(t + k); }
+__device__ __forceinline__ float tex_ld(const hs::h1* __restrict__ t, size_t k) { return hs::ld(t + k, 0); }
+__device__ __forceinline__ float4 tex_ld(const hs::h4* __restrict__ t, size_t k) { return hs::ld(t + k, 0); }
+__device__ __forceinline__ void tex_st(float4* t, size_t k, float4 v) { t[k] = v; }
+__device__ __forceinline__ void tex_st(float* t, size_t k, float v) { t[k] = v; }
+__device__ __forceinline__ void tex_st(hs::h4* t, size_t k, float4 v) { hs::st(t + k, 0, v); }
+__device__ __forceinline__ void tex_st(hs::h1* t, size_t k, float v) { hs::st(t + k, 0, v); }
+// the destination texel of an additive blit (blendFunc(ONE, ONE)): a plain load, the thread overwrites it
+__device__ __forceinline__ float4 dst_ld(const float4* t, size_t k) { return t[k]; }
+__device__ __forceinline__ float4 dst_ld(const hs::h4* t, size_t k) {
+    const hs::h4 v = t[k];
+    const float2 a = __half22float2(v.a), b = __half22float2(v.b);
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+
+// linear_fetch4 of passes.cuh on an fp16 RGBA texture: the same taps, weights and add order
+__device__ __forceinline__ float4 linear_fetch4(const hs::h4* __restrict__ tex, int W, int H, float uvx, float uvy) {
     const float u = uvx * (float)W - 0.5f, v = uvy * (float)H - 0.5f;
     const float fi = floorf(u), fj = floorf(v);
     const float a = u - fi, b = v - fj;
     const int i0 = texel_index(fi, W), i1 = texel_index(fi + 1.0f, W);
     const int j0 = texel_index(fj, H), j1 = texel_index(fj + 1.0f, H);
     const float w00 = (1.0f - a) * (1.0f - b), w10 = a * (1.0f - b), w01 = (1.0f - a) * b, w11 = a * b;
-    return ((w00 * __ldg(&tex[(size_t)j0 * W + i0]) + w10 * __ldg(&tex[(size_t)j0 * W + i1])) +
-            w01 * __ldg(&tex[(size_t)j1 * W + i0])) + w11 * __ldg(&tex[(size_t)j1 * W + i1]);
+    const float4 t00 = tex_ld(tex, (size_t)j0 * W + i0), t10 = tex_ld(tex, (size_t)j0 * W + i1);
+    const float4 t01 = tex_ld(tex, (size_t)j1 * W + i0), t11 = tex_ld(tex, (size_t)j1 * W + i1);
+    float4 r;
+    r.x = ((w00 * t00.x + w10 * t10.x) + w01 * t01.x) + w11 * t11.x;
+    r.y = ((w00 * t00.y + w10 * t10.y) + w01 * t01.y) + w11 * t11.y;
+    r.z = ((w00 * t00.z + w10 * t10.z) + w01 * t01.z) + w11 * t11.z;
+    r.w = ((w00 * t00.w + w10 * t10.w) + w01 * t01.w) + w11 * t11.w;
+    return r;
+}
+
+template <typename T1>
+__device__ __forceinline__ float linear_fetch1(const T1* __restrict__ tex, int W, int H, float uvx, float uvy) {
+    const float u = uvx * (float)W - 0.5f, v = uvy * (float)H - 0.5f;
+    const float fi = floorf(u), fj = floorf(v);
+    const float a = u - fi, b = v - fj;
+    const int i0 = texel_index(fi, W), i1 = texel_index(fi + 1.0f, W);
+    const int j0 = texel_index(fj, H), j1 = texel_index(fj + 1.0f, H);
+    const float w00 = (1.0f - a) * (1.0f - b), w10 = a * (1.0f - b), w01 = (1.0f - a) * b, w11 = a * b;
+    return ((w00 * tex_ld(tex, (size_t)j0 * W + i0) + w10 * tex_ld(tex, (size_t)j0 * W + i1)) +
+            w01 * tex_ld(tex, (size_t)j1 * W + i0)) + w11 * tex_ld(tex, (size_t)j1 * W + i1);
 }
 
 // REPEAT-wrapped LINEAR fetch of the first channel of an RGB (3 floats / texel) texture: the
@@ -40,8 +83,9 @@ __device__ __forceinline__ float linear_fetch_rgb_r_repeat(const float* __restri
 }
 
 // bloomPrefilterShader S:614-631
-__global__ void __launch_bounds__(256) bloom_prefilter_kernel(const float4* __restrict__ dye, int Wd, int Hd,
-                                                              float4* __restrict__ out, int w, int h, float curve0,
+template <typename T4>
+__global__ void __launch_bounds__(256) bloom_prefilter_kernel(const T4* __restrict__ dye, int Wd, int Hd,
+                                                              T4* __restrict__ out, int w, int h, float curve0,
                                                               float curve1, float curve2, float threshold) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= w || j >= h) return;
@@ -51,12 +95,13 @@ __global__ void __launch_bounds__(256) bloom_prefilter_kernel(const float4* __re
     float rq = fminf(fmaxf(br - curve0, 0.0f), curve1);
     rq = (curve2 * rq) * rq;
     const float f = fmaxf(rq, br - threshold) / fmaxf(br, 0.0001f);
-    out[(size_t)j * w + i] = make_float4(c.x * f, c.y * f, c.z * f, 0.0f);
+    tex_st(out, (size_t)j * w + i, make_float4(c.x * f, c.y * f, c.z * f, 0.0f));
 }
 
 // bloomBlurShader S:633-651 / bloomFinalShader S:653-674; add = blendFunc(ONE, ONE) (S:1374-1375)
-__global__ void __launch_bounds__(256) box4_kernel(const float4* __restrict__ src, int ws, int hs,
-                                                   float4* __restrict__ dst, int w, int h, float scale, int add) {
+template <typename T4>
+__global__ void __launch_bounds__(256) box4_kernel(const T4* __restrict__ src, int ws, int hs,
+                                                   T4* __restrict__ dst, int w, int h, float scale, int add) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= w || j >= h) return;
     const float tsx = (float)(1.0 / (double)ws), tsy = (float)(1.0 / (double)hs);
@@ -68,13 +113,14 @@ __global__ void __launch_bounds__(256) box4_kernel(const float4* __restrict__ sr
     s.y = ((((0.0f + L.y) + R.y) + T.y) + B.y) * 0.25f * scale;
     s.z = ((((0.0f + L.z) + R.z) + T.z) + B.z) * 0.25f * scale;
     s.w = ((((0.0f + L.w) + R.w) + T.w) + B.w) * 0.25f * scale;
-    float4* o = dst + (size_t)j * w + i;
-    if (add) { const float4 d = *o; s.x = s.x + d.x; s.y = s.y + d.y; s.z = s.z + d.z; s.w = s.w + d.w; }
-    *o = s;
+    const size_t o = (size_t)j * w + i;
+    if (add) { const float4 d = dst_ld(dst, o); s.x = s.x + d.x; s.y = s.y + d.y; s.z = s.z + d.z; s.w = s.w + d.w; }
+    tex_st(dst, o, s);
 }
 
 // sunraysMaskShader S:676-691 (target = dye.write, like the reference: S:1300)
-__global__ void __launch_bounds__(256) sunrays_mask_kernel(const float4* __restrict__ dye, float4* __restrict__ mask,
+template <typename T4>
+__global__ void __launch_bounds__(256) sunrays_mask_kernel(const T4* __restrict__ dye, T4* __restrict__ mask,
                                                            int Wd, int Hd) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= Wd || j >= Hd) return;
@@ -82,12 +128,13 @@ __global__ void __launch_bounds__(256) sunrays_mask_kernel(const float4* __restr
     float4 c = linear_fetch4(dye, Wd, Hd, uvx, uvy);
     const float br = fmaxf(c.x, fmaxf(c.y, c.z));
     c.w = 1.0f - fminf(fmaxf(br * 20.0f, 0.0f), 0.8f);
-    mask[(size_t)j * Wd + i] = c;
+    tex_st(mask, (size_t)j * Wd + i, c);
 }
 
 // sunraysShader S:693-724
-__global__ void __launch_bounds__(256) sunrays_kernel(const float4* __restrict__ mask, int Wm, int Hm,
-                                                      float* __restrict__ out, int w, int h, float weight) {
+template <typename T4, typename T1>
+__global__ void __launch_bounds__(256) sunrays_kernel(const T4* __restrict__ mask, int Wm, int Hm,
+                                                      T1* __restrict__ out, int w, int h, float weight) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= w || j >= h) return;
     const float Density = 0.3f, Decay = 0.95f, Exposure = 0.7f;
@@ -105,11 +152,12 @@ __global__ void __launch_bounds__(256) sunrays_kernel(const float4* __restrict__
         color = color + (col * illum) * weight;
         illum = illum * Decay;
     }
-    out[(size_t)j * w + i] = color * Exposure;
+    tex_st(out, (size_t)j * w + i, color * Exposure);
 }
 
 // blurShader S:478-494 + blurVertexShader S:461-476 on the one-channel sunrays texture
-__global__ void __launch_bounds__(256) blur3_kernel(const float* __restrict__ src, float* __restrict__ dst, int w, int h,
+template <typename T1>
+__global__ void __launch_bounds__(256) blur3_kernel(const T1* __restrict__ src, T1* __restrict__ dst, int w, int h,
                                                     float tsx, float tsy) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= w || j >= h) return;
@@ -121,13 +169,15 @@ __global__ void __launch_bounds__(256) blur3_kernel(const float* __restrict__ sr
     float sum = c * 0.29411764f;
     sum = sum + l * 0.35294117f;
     sum = sum + r * 0.35294117f;
-    dst[(size_t)j * w + i] = sum;
+    tex_st(dst, (size_t)j * w + i, sum);
 }
 
-// displayShaderSource S:549-612 with SHADING + BLOOM + SUNRAYS over drawColor, premultiplied blend
-__global__ void __launch_bounds__(256) display_full_kernel(const float4* __restrict__ dye, int Wd, int Hd,
-                                                           const float4* __restrict__ bloom, int bw, int bh,
-                                                           const float* __restrict__ sun, int sw, int sh,
+// displayShaderSource S:549-612 with SHADING + BLOOM + SUNRAYS over drawColor, premultiplied blend;
+// the target is fp32 in both storage modes (the unquantised frame fluid_render returns)
+template <typename T4, typename T1>
+__global__ void __launch_bounds__(256) display_full_kernel(const T4* __restrict__ dye, int Wd, int Hd,
+                                                           const T4* __restrict__ bloom, int bw, int bh,
+                                                           const T1* __restrict__ sun, int sw, int sh,
                                                            const float* __restrict__ dither, int dw, int dh,
                                                            float4* __restrict__ out, int w, int h, float br_, float bg_,
                                                            float bb_, int bg_mode, float aspect, float4 ts) {
